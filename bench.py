@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo (CUDA, sm_100a)
     python bench.py --impl reference --gpus N ...            # the reference's CPU path (oracle port)
+    python bench.py ... --dump-outputs DIR                    # also save the last timed step's digests as DIR/*.npy
 
 A "step" is one full digest of the blob: leaf SHA-256 over every 16 KiB of blob bytes, the tree levels above them up
 to the 8 MiB chunk-digest list, the levels above that, and the root (modelx.tree.v1, DESIGN.md section 3 -- a NEW
@@ -65,7 +66,22 @@ def parse_args():
     ap.add_argument("--compat5-blob-mb", type=float, default=128.0)
     ap.add_argument("--compat3-shards", type=int, default=32)
     ap.add_argument("--compat3-shard-gb", type=float, default=0.5)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the chunk digests and the root of the last timed step to DIR/<name>.npy (float32), so "
+                         "that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.dump_outputs and args.steps < 1:
+        ap.error("--dump-outputs needs --steps >= 1")
+    return args
+
+
+def dump_outputs(d, chunk_list: bytes, root: bytes):
+    """The digests a caller of the timed path receives, one byte per float32 element (exact for 0..255): the
+    32-byte chunk digests as an (nchunks, 32) array and the 32-byte root.  The 100 GB blob has 11,921 chunks, 1.5 MB."""
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    np.save(os.path.join(d, "chunk_digests.npy"), np.frombuffer(chunk_list, dtype=np.uint8).reshape(-1, 32).astype(np.float32))
+    np.save(os.path.join(d, "root.npy"), np.frombuffer(root, dtype=np.uint8).astype(np.float32))
 
 
 def load_peaks():
@@ -405,6 +421,8 @@ def run_b200(args):
     value = size * args.steps / (ms_max * 1e-3) / GB
     root_dev = bytes(d_root.cpu().numpy().tobytes())
     chunk_list_dev = bytes((d_all if world > 1 else d_local).cpu().numpy().tobytes())[:nchunks * 32]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, chunk_list_dev, root_dev)
     launches = st1["kernel_launches"] - st0["kernel_launches"]
 
     # roofline of the dominant kernel: the leaf-level launch (reads every blob byte once)
